@@ -20,8 +20,12 @@ configs[3] at its stated length (50 waypoints, CartVel + LVS continuous collisio
 Every step uses a different synthetic batch (seed = f(step, rank)), so nothing is cached between timed iterations; the
 working set of one step (~0.6 GB of convexification rows + QP workspace at B=1024 with collision) is larger than L2.
 --scaling strong splits ONE global batch (--batch) over the ranks instead of giving every rank its own.
+--dump-outputs DIR writes the results of the last timed step of the `value` leg (what tb200_fetch_results hands the
+caller) as DIR/<name>.npy in float64, so that two builds run with the same arguments can be compared output for output.
+The benchmark writes nothing into the source tree.
 """
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -31,6 +35,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -143,6 +148,7 @@ class ClockSampler:
         try:
             self.proc = subprocess.Popen(["nvidia-smi", f"--query-gpu={q}", "--format=csv,noheader,nounits", "-i",
                                           str(self.index), "-lms", "100"], stdout=subprocess.PIPE, text=True)
+            atexit.register(self.proc.kill)  # the sampler must not outlive a run that raises before stop()
             threading.Thread(target=self._read, daemon=True).start()
         except OSError:
             self.proc = None
@@ -166,7 +172,7 @@ class ClockSampler:
 def oracle_module():
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     import oracle_lib  # the CPU legs: the oracle is the timed CPU path here, never part of the product
-    oracle_lib.build()
+    oracle_lib.lib()  # loads the library build() made; no make run, so a read-only tree works
     return oracle_lib
 
 
@@ -244,6 +250,26 @@ def measured_traffic(config):
         return None
 
 
+DUMP_BUDGET = 64 << 20
+
+
+def dump_outputs(out_dir, res, budget=DUMP_BUDGET):
+    """Writes the per-trajectory result arrays of one solve as out_dir/<name>.npy (float64).  Above `budget` bytes a fixed
+    sample of trajectories (numpy default_rng(0), in batch order) is written instead, with their batch indices in
+    trajectory_index.npy."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in res.items() if isinstance(v, np.ndarray)}
+    B = len(arrays["status"])
+    per_traj = sum(a.nbytes for a in arrays.values()) / B + 8
+    n = min(B, int((budget - 128 * (len(arrays) + 1)) // per_traj))  # 128: one .npy header per file
+    if n < B:
+        idx = np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+        arrays["trajectory_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -260,7 +286,13 @@ def main():
     ap.add_argument("--cpu-repeats", type=int, default=3, help="cpu_baseline: best of this many runs")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step as DIR/<name>.npy "
+                                                          f"(float64, at most {DUMP_BUDGET >> 20} MB in all)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs writes the results of the CUDA path (--impl cuda)")
     if args.batch <= 0:
         args.batch = DEFAULT_BATCH[args.config]
 
@@ -335,6 +367,7 @@ def main():
         # launch writes ~135 MB > L2): the launch the roofline below is quoted on
         ktm.append(prob.convexify_timed(res["x"]))
     fence()
+    resident_last = res
     # ---- end-to-end leg: K steps through the public API with host buffers, one fence on each side -------------------
     t0 = time.perf_counter()
     e2e_conv, h2d, d2h, last = 0, 0, 0, None
@@ -347,6 +380,9 @@ def main():
     e2e_s = time.perf_counter() - t0
     clocks = sampler.stop() if rank == 0 else None
     fence()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs if world == 1 else os.path.join(args.dump_outputs, f"rank{rank}"), resident_last,
+                     DUMP_BUDGET // world)
 
     def reduce(v, op):
         if world == 1:
